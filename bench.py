@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — reads/sec of the `coverm contig|genome --bam-files` coverage hot path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|ns|3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|ns|3] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (`--config`, all synthetic, SURVEY.md §8d; the default is BASELINE.json configs[1]):
@@ -22,6 +22,14 @@ One "step" = one pass of the hot path over one sample.
   roofline / cpu_baseline as described in DESIGN.md (Measurement).
 `--impl reference` times the CPU restatement of the reference (oracle/, all host threads for BGZF inflate, the record loop
 single-threaded exactly as the reference's) on the SAME file and command; one step = one full run.
+
+`--dump-outputs DIR` writes what the last timed step returned, as float64 .npy files (at most 64 MB), so that two builds can be
+compared output for output; the workload's records depend only on the arguments (`--seed` included):
+  contig_stats.npy    the device step's per-contig table (cmb_contig_stats in declaration order, without `hist_offset` and
+                      `reserved`), one row per contig of contig_stats_rows.npy (all contigs, or a fixed sample seeded by --seed);
+                      sum_identity_primary / sum_identity_nonsupp are f64 sums of atomic adds: their last bits vary run to run
+  table.npy           the numbers of the last e2e step's printed table (header and name column dropped), one row per table row
+                      of table_rows.npy (same sampling); with --impl reference the oracle's table of its last run
 """
 import argparse
 import json
@@ -161,6 +169,50 @@ def run_oracle(cfg, bam, threads, runs, warmup):
     return sum(times) / len(times), out
 
 
+DUMP_BYTES = 64 << 20  # everything --dump-outputs writes, row indices included
+
+
+def sample_rows(n, row_bytes, budget, seed):
+    """Indices of the rows of an n-row output that fit in `budget` bytes: all of them, or a sorted sample fixed by `seed`."""
+    import numpy as np
+    cap = max(1, budget // row_bytes)
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, cap, replace=False))
+
+
+def device_table(ptr, n_rows):
+    """The n_rows cmb_contig_stats rows at device address `ptr` (cmb_end_sample_device), copied into a host array."""
+    import numpy as np
+    import torch
+    from coverm_b200 import ContigStats
+    cai = {"shape": (n_rows * C_sizeof(ContigStats),), "typestr": "|u1", "data": (ptr, False), "version": 2}
+    rows = torch.as_tensor(type("DeviceRows", (), {"__cuda_array_interface__": cai})(), device="cuda")
+    return rows.cpu().numpy().view(np.dtype(ContigStats))
+
+
+def dump_outputs(out_dir, seed, table_text, stats=None):
+    """--dump-outputs: the printed table's numbers and, for our arm, the device step's per-contig table (module docstring)."""
+    import numpy as np
+    from coverm_b200 import ContigStats
+    arrays = {}
+    if stats is not None:
+        # hist_offset is where K3's atomic counter placed the row's histogram pairs: it follows the order the rows finished in
+        fields = [f for f, _ in ContigStats._fields_ if f not in ("hist_offset", "reserved")]
+        rows = sample_rows(len(stats), 8 * (len(fields) + 1), DUMP_BYTES // 3, seed)
+        arrays["contig_stats"] = np.stack([stats[f][rows].astype(np.float64) for f in fields], axis=1)
+        arrays["contig_stats_rows"] = rows.astype(np.float64)
+    lines = table_text.splitlines()[1:]
+    table = np.array([[float(x) for x in l.split("\t")[1:]] for l in lines], dtype=np.float64).reshape(len(lines), -1)
+    rows = sample_rows(len(table), 8 * (table.shape[1] + 1), DUMP_BYTES // 2, seed)
+    arrays["table"] = table[rows]
+    arrays["table_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"wrote {', '.join(f'{n}.npy {a.shape}' for n, a in arrays.items())} to {out_dir}")
+
+
 def cpu_baseline_entry(records, sec, threads, runs, what):
     return {"value": records / sec, "unit": "reads/s", "cores": threads, "kind": "port",
             "sample": f"{what}; oracle/coverm_oracle -t {threads}: {threads} BGZF inflate threads, single-threaded record loop + one "
@@ -179,14 +231,17 @@ def main():
     ap.add_argument("--contigs", type=int, default=0, help="override the workload's contig count")
     ap.add_argument("--reads", type=int, default=0, help="override the workload's read count")
     ap.add_argument("--seed", type=int, default=20260925)
-    ap.add_argument("--ref-budget-s", type=float, default=420.0, help="--impl reference: wall-clock budget for all of its runs")
     ap.add_argument("--e2e-steps", type=int, default=0, help="timed e2e steps (default: --steps)")
     ap.add_argument("--skip-cpu-baseline", action="store_true", help="no oracle run (then no parity check and no cpu_baseline)")
     ap.add_argument("--skip-cold-cli", action="store_true")
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="N > 1: strong = one sample range-partitioned by contig over the N GPUs (default); weak = N samples, one per GPU")
     ap.add_argument("--workdir", default=os.environ.get("CMB_BENCH_DIR", "/tmp/coverm_b200_bench"))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     args.contigs = args.contigs or cfg["contigs"]
     args.reads = args.reads or cfg["reads"]
@@ -217,18 +272,16 @@ def main():
             return
         bam = os.path.join(args.workdir, f"sample_c{args.config}_r0_{args.contigs}_{args.reads}.bam")
         info = gen_bam(bam, cfg, args.contigs, args.reads, args.seed, ncpu)
-        t0 = time.perf_counter()
         warm = 0
         if args.warmup > 0:  # one untimed warm-up run (page cache, CPU clocks); more would only repeat it
             run_oracle(cfg, bam, ncpu, 1, 0)
             warm = 1
         times = []
-        while len(times) < args.steps:
-            elapsed = time.perf_counter() - t0
-            est = max(times) if times else (elapsed if warm else 0.0)
-            if times and elapsed + est > args.ref_budget_s:
-                break
-            times.append(run_oracle(cfg, bam, ncpu, 1, 0)[0])
+        for _ in range(args.steps):
+            sec, out = run_oracle(cfg, bam, ncpu, 1, 0)
+            times.append(sec)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, args.seed, out)
         steps = len(times)
         sec = sum(times) / steps
         cpu = cpu_baseline_entry(info["records"], sec, ncpu, steps, "the full workload file")
@@ -239,8 +292,7 @@ def main():
                 "config": workload_config(cfg, args, info, args.gpus, args.scaling),
                 "cpu_baseline": cpu,
                 "e2e": {"value": cpu["value"], "unit": "reads/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-                "note": f"each step is one full `coverm` run on the whole file ({sec:.1f} s); steps/warmup are what actually ran "
-                        f"inside a {args.ref_budget_s:.0f} s budget"}
+                "note": f"each step is one full `coverm` run on the whole file ({sec:.1f} s); at most one warm-up run"}
         emit(line)
         return
 
@@ -341,9 +393,10 @@ def main():
     def device_step():
         ctx.begin_sample()
         ctx.submit_device_batch(batch, n_rec, n_iv)
-        ctx.end_sample_device()  # K1c/K1b/K2/K3 + error check (stream-synchronous)
+        rows = ctx.end_sample_device()  # K1c/K1b/K2/K3 + error check (stream-synchronous); the table stays in HBM
         if strong:
             ctx.allgather_stats(cuts)  # the collective of the path, on the same stream (NCCL broadcasts of each rank's row range)
+        return rows
 
     sampler = ClockSampler(local_rank)
     n_warm = max(3, args.warmup)
@@ -360,7 +413,7 @@ def main():
         ev0.record()
     launches = 0
     for _ in range(args.steps):
-        device_step()
+        dev_rows = device_step()
         tm = ctx.timing()
         k0_ms.append(tm["ms_zero"]); k1_ms.append(tm["ms_accumulate"]); k2_ms.append(tm["ms_scan"]); k3_ms.append(tm["ms_finalize"])
         dev_ms.append(tm["ms_total"])
@@ -371,6 +424,8 @@ def main():
     wall_ms = (time.perf_counter() - t_wall) * 1e3
     barrier()
     event_ms = ev0.elapsed_time(ev1)  # the gather is enqueued on the same stream: the events bracket it too
+    # the last step's table, before the e2e arm's next sample overwrites it
+    dumped_stats = device_table(dev_rows, n_contigs) if args.dump_outputs and rank == 0 else None
     step_ms = max_over_ranks(event_ms / args.steps)
     total_reads = float(file_records) if strong else sum_over_ranks(float(n_rec))
     value = total_reads / (step_ms * 1e-3)
@@ -455,6 +510,8 @@ def main():
             log(f"PARITY FAILURE on the full file: {len(gl)} vs {len(ol)} lines; first differences {diff}")
     sess.close()
 
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, args.seed, e2e_out, dumped_stats)
     if rank == 0:
         scaling = "strong" if strong else "weak"
         config = workload_config(cfg, args, info, world, scaling)

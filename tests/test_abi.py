@@ -3,12 +3,25 @@ version, and refuses to run without a CUDA device (no CPU fallback).  No GPU nee
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 
 import pytest
+import torch
 
 import coverm_b200
 from case_runner import ROOT
+
+
+def _build_nvcc():
+    """The nvcc coverm_b200/csrc/Makefile compiles with: $NVCC, else the Makefile's default."""
+    mk = open(os.path.join(ROOT, "coverm_b200", "csrc", "Makefile")).read()
+    nvcc = os.environ.get("NVCC") or re.search(r"^NVCC \?= *(\S+)", mk, re.M).group(1)
+    return shutil.which(nvcc) or nvcc
+
+
+# the toolkit that built the library disassembles it
+CUOBJDUMP = os.path.join(os.path.dirname(_build_nvcc()), "cuobjdump")
 
 
 @pytest.fixture(scope="module")
@@ -41,7 +54,7 @@ def test_abi_version_and_struct_sizes(lib):
 
 
 def test_kernels_are_sm_100a_with_tma(lib):
-    out = subprocess.run(["cuobjdump", "-sass", coverm_b200.LIB_PATH], capture_output=True, text=True).stdout
+    out = subprocess.run([CUOBJDUMP, "-sass", coverm_b200.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
     assert "UTMALDG" in out, "K2 must stage its tiles with TMA (cp.async.bulk.tensor)"
     for k in ("k1_filter_accumulate", "k1b_local", "k1b_apply", "k2_scan_reduce", "k3_finalize", "kd_inflate", "kd_inflate_g8", "kd_guess", "kd_walk",
@@ -49,7 +62,8 @@ def test_kernels_are_sm_100a_with_tma(lib):
         assert k in out
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="a GPU is present")
+# any visible CUDA device: its device node need not be /dev/nvidia0
+@pytest.mark.skipif(torch.cuda.is_available(), reason="a CUDA device is visible")
 def test_fails_loudly_without_a_gpu(lib):
     h = ctypes.c_void_p()
     cfg = coverm_b200.DeviceCfg(0, 1024, 2048, 2)

@@ -2,10 +2,7 @@
 #pragma once
 
 
-#ifndef CMB_SPAN
-#define CMB_SPAN 32
-#endif
-constexpr uint32_t SPAN = CMB_SPAN;             // elements per thread span; contig alignment (16 or 32)
+constexpr uint32_t SPAN = 32;                   // elements per thread span; contig alignment
 constexpr uint32_t K2_THREADS = 8192 / SPAN;
 constexpr uint32_t CHUNK = SPAN * K2_THREADS;   // 8192 elements = 32 KB
 constexpr uint32_t CHUNK_BYTES = CHUNK * 4;
@@ -17,12 +14,6 @@ constexpr uint32_t CHUNK_ROWS = CHUNK / ROW_ELEMS;  // 256
 #endif
 constexpr uint32_t K2_STAGES = CMB_K2_STAGES;
 constexpr uint32_t K2_WARPS = K2_THREADS / 32;  // 16
-#ifndef CMB_K2_COOP
-#define CMB_K2_COOP 0  // K2 experiment: warp-cooperative handling of the non-empty spans (measured SLOWER: 2.85 vs 2.66 ms on config 2)
-#endif
-#ifndef CMB_K2_STATIC
-#define CMB_K2_STATIC 1  // K2: static chunk schedule, chunk metadata requested an iteration ahead (0 = dynamic tickets; 2.64 vs 2.69 ms)
-#endif
 #ifndef CMB_HIST_SLOTS
 #define CMB_HIST_SLOTS 8
 #endif
@@ -51,9 +42,6 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   asm volatile(

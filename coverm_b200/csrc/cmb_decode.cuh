@@ -2,12 +2,13 @@
 // boundaries and reduces every record to the cmb_read_batch tuple K1 consumes.  Replaces, for the stream (non-pair) path,
 // htslib's bgzf_read + bam_read1 behind BamFileNamedReader::read (bam_generator.rs:103-134).
 //
-//   KD1 kd_inflate   one warp per BGZF block (RFC 1951); the default is kd_inflate_g8 (cmb_decode_g8.cuh, four blocks per
-//                    warp), this one-stream-per-warp form stays selectable with CMB_INFLATE_G8=0.  All 32 lanes run the decoder redundantly (uniform control
-//                    flow), which turns the lanes into resources: the compressed bytes are held as a 2 x 128-byte
-//                    register window fetched with coalesced loads and read with shuffles; length/distance base tables
-//                    live one entry per lane; LZ77 matches are copied by all lanes; Huffman tables (10-bit root + 5-bit
-//                    subtables, u16 entries) are built cooperatively in shared memory.  The block's CRC-32 is then
+//   KD1 kd_inflate   one warp per BGZF block (RFC 1951); kd_inflate_g8 (cmb_decode_g8.cuh) takes four blocks per warp and
+//                    kd_inflate_t1 (cmb_decode_t1.cuh) one block per lane; this form is CMB_INFLATE=w1 (see inflate_kind).
+//                    All 32 lanes run the decoder redundantly (uniform control flow), which turns the lanes into
+//                    resources: the compressed bytes are held as a 2 x 128-byte register window fetched with
+//                    coalesced loads and read with shuffles; length/distance base tables live one entry per lane;
+//                    LZ77 matches are copied by all lanes; Huffman tables (10-bit root + 5-bit subtables, u16
+//                    entries) are built cooperatively in shared memory.  The block's CRC-32 is then
 //                    checked against the BGZF footer (per-lane slices combined in GF(2)).
 //   KD2 kd_guess     one warp per block: the first offset >= the block start from which a chain of plausible record
 //                    headers runs (records straddle blocks freely).
@@ -60,8 +61,7 @@ struct InflateArgs {
   // (written by the copy stream after the window's bytes; NULL = everything is resident)
   const uint32_t* block_window;
   const uint32_t* ready;
-  uint32_t lane_limit;    // kd_inflate_t1: lanes per warp that take blocks (0 = all 32)
-  uint32_t static_first;  // kd_inflate_t1: the first block of every lane is dealt out column-wise (see the kernel)
+  uint32_t lane_limit;  // kd_inflate_t1: lanes per warp that take blocks (0 = all 32)
   // optional indirection: ticket t in [b0, b1) names block block_list[t] (second pass over the blocks the first declined)
   const uint32_t* block_list;
   uint8_t* scratch;  // kd_inflate_t1: 160 bytes per BGZF block (indexed by block number)

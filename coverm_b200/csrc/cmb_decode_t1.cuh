@@ -177,22 +177,10 @@ __global__ void __launch_bounds__(T1_THREADS, 5) kd_inflate_t1(const InflateArgs
   // With fewer blocks than the grid has lanes, only the first lane_limit lanes of every warp work: the blocks spread over all
   // the warps instead of filling the first ones.
   if (a.lane_limit && (threadIdx.x & 31) >= a.lane_limit) return;
-  // static_first (experiment, off by default): the first round is dealt out column-wise -- lane j of warp w starts with block
-  // j * n_warps + w, so a warp's lanes hold blocks spread evenly over the file instead of neighbouring ones.  Measured: no
-  // shorter tail on a streamed file, slower on a resident one (the neighbours' locality is lost).
-  const uint32_t n_warps = gridDim.x * (T1_THREADS / 32);
-  bool first_round = a.static_first != 0;
-  const uint32_t static_round = first_round ? (a.lane_limit ? a.lane_limit : 32u) * n_warps : 0u;
   for (;;) {
     // ------------------------------------------------------------------ a new block
     if (state == IDLE) {
-      uint32_t tk;
-      if (first_round) {  // lane j of warp w starts with block j * n_warps + w: one block of every stretch of the file per warp
-        tk = (threadIdx.x & 31) * n_warps + (blockIdx.x * (T1_THREADS / 32) + (threadIdx.x >> 5));
-        first_round = false;
-      } else {
-        tk = static_round + atomicAdd(a.ticket, 1u);
-      }
+      const uint32_t tk = atomicAdd(a.ticket, 1u);
       if (tk >= a.b1 - a.b0) return;
       b = a.block_list ? a.block_list[tk] : a.b0 + tk;
       spins = 0;

@@ -144,7 +144,7 @@ struct cmb_ctx {
   int32_t *d_tail_sum = nullptr, *d_carry_in = nullptr;
   int2* d_block_agg = nullptr;
   cmb_contig_stats* d_rows = nullptr;
-  uint32_t* d_counters = nullptr;  // [0] error flags, [1] ticket, [2] rec_count, [3] ovf_count, [4..5] pair_count (u64),
+  uint32_t* d_counters = nullptr;  // [0] error flags, [1] unused, [2] rec_count, [3] ovf_count, [4..5] pair_count (u64),
                                    // [6..7] kept tid range of the exclusive records (K1Args::kept_range)
   uint32_t kept_range[2] = {0, 0};  // host copy after cmb_end_sample*
   // multi-GPU (cmb_comm_*): one NCCL communicator per ctx, collectives on the ctx stream
@@ -173,8 +173,7 @@ struct cmb_ctx {
   uint32_t *d_gene_first = nullptr, *d_gene_start = nullptr, *d_gene_end = nullptr, *d_gene_maxlen = nullptr, *d_contig_len32 = nullptr;
   uint8_t* d_contig_seen = nullptr;
   CUtensorMap tmap{};
-  bool arena_dirty = true;
-  bool clean_as_you_go = true;
+  bool arena_dirty = true;  // cmb_begin_sample must zero the arena: only a completed K2 leaves it clean
   // params
   cmb_params params{};
   cmb_filter_mode mode{};
@@ -195,7 +194,7 @@ struct cmb_ctx {
     uint32_t *d_clen = nullptr, *d_isize = nullptr, *d_status = nullptr, *d_nrec = nullptr, *d_ncig = nullptr, *d_dirty = nullptr;
     size_t blocks_cap = 0;
     uint8_t* d_t1_scratch = nullptr;  // kd_inflate_t1: code-length scratch, 160 B per block
-    uint32_t* d_tickets = nullptr;  // [0] block ticket, [1 + w] window w has arrived
+    uint32_t* d_tickets = nullptr;  // [0] block ticket, [1 + w] arrival flag: window w has been copied
     size_t tickets_cap = 0;
     uint32_t* d_block_window = nullptr;
     size_t block_window_cap = 0;
@@ -229,9 +228,6 @@ struct cmb_ctx {
     std::vector<void*> pinned;
     std::vector<cudaStream_t> streams;
     std::vector<cudaEvent_t> slot_events, done_events;
-    std::vector<cudaStream_t> cstreams;      // per-window inflate launches (CMB_INFLATE=t1): kernels of different windows overlap
-    std::vector<cudaEvent_t> window_events;  // window w has been copied
-    std::vector<cudaEvent_t> cstream_done;
     cudaEvent_t ev[6]{};
     bool have_events = false;
   } dec;
@@ -394,9 +390,9 @@ int launch_k1(cmb_ctx* c, const cmb_read_batch& b, uint32_t n_records, uint32_t 
   return CMB_OK;
 }
 
-template <bool HIST, bool CLEAN>
+template <bool HIST>
 int launch_k2_variant(cmb_ctx* c, const K2Args& a) {
-  auto kern = k2_scan_reduce<HIST, CLEAN>;
+  auto kern = k2_scan_reduce<HIST>;
   constexpr uint32_t smem_bytes = HIST ? K2_SMEM_BYTES_HIST : K2_SMEM_BYTES_NOHIST;
   CU_TRY(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
   int occ = 0;
@@ -428,18 +424,16 @@ int run_end_of_sample(cmb_ctx* c) {
   K2Args a{};
   a.off_span = c->d_off_span; a.len = c->d_len; a.chunk_first = c->d_chunk_first; a.carry_in = c->d_carry_in;
   a.rows = c->d_rows; a.tid_begin = c->tid_begin; a.n_local = c->n_local; a.n_chunks = c->n_chunks; a.excl = excl;
-  a.ticket = c->d_counters + 1; a.arena = c->d_arena;
+  a.arena = c->d_arena;
   a.rec = c->d_rec; a.rec_capacity = c->rec_capacity; a.rec_count = c->d_counters + 2;
   a.warp_table = c->d_warp_table; a.ovf = c->d_ovf; a.ovf_head = c->d_ovf_head; a.ovf_capacity = c->ovf_capacity; a.ovf_count = c->d_counters + 3;
   a.error_flags = c->d_counters + 0;
   if (hist) CU_TRY(c, cudaMemsetAsync(c->d_ovf_head, 0xff, 4ull * c->n_chunks, c->stream));
   CU_TRY(c, cudaEventRecord(c->ev[3], c->stream));
-  int rc;
-  if (hist) rc = c->clean_as_you_go ? launch_k2_variant<true, true>(c, a) : launch_k2_variant<true, false>(c, a);
-  else rc = c->clean_as_you_go ? launch_k2_variant<false, true>(c, a) : launch_k2_variant<false, false>(c, a);
+  const int rc = hist ? launch_k2_variant<true>(c, a) : launch_k2_variant<false>(c, a);
   if (rc) return rc;
   c->timing.k2_launches = 1;
-  c->arena_dirty = !c->clean_as_you_go;
+  c->arena_dirty = false;  // K2 re-zeroed every delta it read
   CU_TRY(c, cudaEventRecord(c->ev[4], c->stream));
   if (hist) {
     K3Args k{};
@@ -565,8 +559,6 @@ int cmb_create(const cmb_device_cfg* cfg, cmb_ctx** out) {
   c->block_minmax_capacity = 1u << 16;
   CREATE_TRY(cudaMalloc(&c->d_block_minmax, sizeof(int2) * (size_t)c->block_minmax_capacity));
   CREATE_TRY(cudaMalloc(&c->d_block_xrange, sizeof(int2) * (size_t)c->block_minmax_capacity));
-  const char* env = getenv("CMB_CLEAN_AS_YOU_GO");
-  if (env && env[0] == '0') c->clean_as_you_go = false;
   *out = c;
   return CMB_OK;
 }
@@ -602,9 +594,6 @@ void cmb_destroy(cmb_ctx* c) {
     for (auto st : d.streams) cudaStreamDestroy(st);
     for (auto e : d.slot_events) cudaEventDestroy(e);
     for (auto e : d.done_events) cudaEventDestroy(e);
-    for (auto st : d.cstreams) cudaStreamDestroy(st);
-    for (auto e : d.window_events) cudaEventDestroy(e);
-    for (auto e : d.cstream_done) cudaEventDestroy(e);
     if (d.have_events)
       for (auto e : d.ev) cudaEventDestroy(e);
   }
@@ -1176,12 +1165,11 @@ constexpr size_t DEC_SLACK = 1024;
 constexpr size_t DEC_FRONT = 256;              // readable bytes in front of the first uploaded block (the bit readers align down)
 constexpr uint64_t DEC_TAIL_BYTES = 4u << 20;  // ranged decode: inflated bytes kept beyond the range for its last straddling record
 
-// Launch the inflate kernel over blocks [a.b0, a.b1).  CMB_INFLATE selects the first-pass kernel: t1 (default: one thread
-// per block + kd_crc32), g8 (four blocks per warp) or w1 (one block per warp, also the second pass over declined blocks).
-// First-pass inflate kernel: 0 = kd_inflate_t1 (a thread per block), 1 = kd_inflate_g8 (four blocks per warp), 2 = kd_inflate (a
-// warp per block).  t1 has the higher THROUGHPUT (its ~75 000 streams in flight need that many blocks) but every block takes
-// ~50 ms however few there are; g8 finishes a block in ~20 ms.  So the choice follows the number of blocks: a whole 10 M-read
-// file (46 000 blocks) goes to t1, a rank's share of it on 4 or 8 GPUs to g8.  CMB_INFLATE=t1|g8|w1 overrides.
+// First-pass inflate kernel: 0 = kd_inflate_t1 (a thread per block, then kd_crc32), 1 = kd_inflate_g8 (four blocks per warp),
+// 2 = kd_inflate (a warp per block; it is also the second pass over the blocks the first pass declined).  t1 has the higher
+// THROUGHPUT (its ~75 000 streams in flight need that many blocks) but every block takes ~50 ms however few there are; g8
+// finishes a block in ~20 ms.  So the choice follows the number of blocks: a whole 10 M-read file (46 000 blocks) goes to t1,
+// a rank's share of it on 4 or 8 GPUs to g8.  CMB_INFLATE=t1|g8|w1 forces one kernel, e.g. to run each of them on a small file.
 constexpr uint32_t T1_MIN_BLOCKS = 28000;
 int inflate_kind(uint32_t n_blocks) {
   static const int forced = [] {
@@ -1189,24 +1177,13 @@ int inflate_kind(uint32_t n_blocks) {
     if (e && !strcmp(e, "t1")) return 0;
     if (e && !strcmp(e, "g8")) return 1;
     if (e && !strcmp(e, "w1")) return 2;
-    if (getenv("CMB_INFLATE_G8") && getenv("CMB_INFLATE_G8")[0] == '0') return 2;
     return -1;
   }();
   if (forced >= 0) return forced;
-  static const uint32_t min_blocks = [] {
-    const char* e = getenv("CMB_T1_MIN_BLOCKS");  // experiment knob
-    return e ? (uint32_t)atol(e) : T1_MIN_BLOCKS;
-  }();
-  return n_blocks >= min_blocks ? 0 : 1;
+  return n_blocks >= T1_MIN_BLOCKS ? 0 : 1;
 }
-// Default: ONE persistent launch whose threads poll the windows' arrival flags (bounded wait), so that every SM has work as soon
-// as the first window is in.  CMB_INFLATE_WINDOWS=1 (t1 only) launches per copied window instead, stream-ordered behind the
-// window's copy -- nothing on the device then waits for data, which tools that serialise streams (ncu, compute-sanitizer)
-// need; with the default 8 hardware queues (CUDA_DEVICE_MAX_CONNECTIONS) those launches overlap poorly, hence not the default.
-bool inflate_per_window() {
-  static const bool v = getenv("CMB_INFLATE_WINDOWS") && getenv("CMB_INFLATE_WINDOWS")[0] == '1';
-  return v;
-}
+// Two launch disciplines for the inflate stage.  Persistent (the default): ONE launch before the copies, whose threads poll
+// the windows' arrival flags (bounded wait), so that every SM has work as soon as the first window is in.
 // Serial mode: copy everything, then ONE inflate launch ordered behind the copies on the context stream -- no flags, nothing on
 // the device waits for anything.  Used for files of a single window (nothing to overlap), on request (CMB_INFLATE_SERIAL=1),
 // and when a CUDA tool is injected into the process (ncu, compute-sanitizer: they serialise kernels against the other streams,
@@ -1228,6 +1205,7 @@ int launch_crc32(cmb_ctx* c, const InflateArgs& a, cudaStream_t st) {
   CU_TRY(c, cudaGetLastError());
   return CMB_OK;
 }
+// Launch the first-pass (or, with first_pass false or a block list, the second-pass) inflate kernel over blocks [a.b0, a.b1).
 // *crc_pending (when given) is set instead of launching kd_crc32: the caller launches it once nothing else has to get past it
 // in the hardware queue (a kernel waiting for its predecessor blocks the queue for every stream that shares it).
 int launch_inflate(cmb_ctx* c, const InflateArgs& a, cudaStream_t st, bool first_pass = true, bool* crc_pending = nullptr) {
@@ -1238,19 +1216,11 @@ int launch_inflate(cmb_ctx* c, const InflateArgs& a, cudaStream_t st, bool first
     CU_TRY(c, cudaFuncSetAttribute(kd_inflate_t1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM_BYTES));
     // every resident warp takes part; with fewer blocks than lanes, each warp works with its first `lanes` lanes only
     const uint32_t max_grid = (uint32_t)c->sm_count * 5, warps = max_grid * (T1_THREADS / 32);
-    uint32_t lanes = std::min<uint32_t>(32, std::max<uint32_t>(1, (nb + warps - 1) / warps));
-    static const int lanes_forced = [] { const char* e = getenv("CMB_T1_LANES"); return e ? atoi(e) : 0; }();  // experiment knob
-    if (lanes_forced > 0) lanes = std::min<uint32_t>(32, (uint32_t)lanes_forced);
+    const uint32_t lanes = std::min<uint32_t>(32, std::max<uint32_t>(1, (nb + warps - 1) / warps));
     const uint32_t per_cta = lanes * (T1_THREADS / 32);
-    uint32_t grid = std::min<uint32_t>((nb + per_cta - 1) / per_cta, max_grid);
-    if (const char* cap = getenv("CMB_T1_MAX_CTAS")) grid = std::max<uint32_t>(1, std::min<uint32_t>(grid, (uint32_t)atoi(cap)));  // experiment knob: fewer live streams
+    const uint32_t grid = std::min<uint32_t>((nb + per_cta - 1) / per_cta, max_grid);
     InflateArgs at = a;
     at.lane_limit = lanes;
-    // experiment knob, measured and left off: dealing the first round out column-wise (a warp's lanes hold blocks spread over
-    // the file) does not shorten the tail of a streamed file (94 vs 93 ms on config 2) and costs locality when the file is
-    // resident (82 vs 49 ms)
-    static const bool columns = getenv("CMB_T1_COLUMNS") && getenv("CMB_T1_COLUMNS")[0] == '1';
-    at.static_first = (!a.block_list && columns) ? 1u : 0u;
     kd_inflate_t1<<<grid, T1_THREADS, T1_SMEM_BYTES, st>>>(at);
     CU_TRY(c, cudaGetLastError());
     if (crc_pending) *crc_pending = true;
@@ -1279,6 +1249,20 @@ int dec_grow(cmb_ctx* c, T*& p, size_t& cap, size_t need, size_t extra_bytes = 0
   CU_TRY(c, cudaMalloc(&p, want * sizeof(T) + extra_bytes));
   cap = want;
   return CMB_OK;
+}
+
+// zlib's raw inflate of BGZF block b into tmp (grown to fit); true when the stream ends with exactly the block's isize bytes
+bool zlib_inflate_block(z_stream& zs, const cmb_bgzf_input* in, uint32_t b, std::vector<uint8_t>& tmp, int* zrc = nullptr) {
+  const uint32_t isz = in->block_isize[b];
+  if (tmp.size() < isz) tmp.resize(isz);
+  inflateReset(&zs);
+  zs.next_in = const_cast<Bytef*>(in->data + in->block_coffset[b]);
+  zs.avail_in = in->block_clen[b];
+  zs.next_out = tmp.data();
+  zs.avail_out = isz;
+  const int rc = inflate(&zs, Z_FINISH);
+  if (zrc) *zrc = rc;
+  return rc == Z_STREAM_END && zs.avail_out == 0;
 }
 }  // namespace
 
@@ -1440,7 +1424,6 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
   if (const char* lim = getenv("CMB_DECODE_MEM_LIMIT_MB")) {  // testing aid: behave as if the device had this much room
     if (((byte_hi - byte_lo) + (total - u_lo)) >> 20 > strtoull(lim, nullptr, 10)) return CMB_E_NOMEM;
   }
-  size_t dummy_cap;
   int rc;
   if ((rc = dec_grow(c, d.d_comp, d.comp_cap, (size_t)(byte_hi - byte_lo) + DEC_FRONT + DEC_SLACK))) return rc;
   if ((rc = dec_grow(c, d.d_inflated, d.infl_cap, (size_t)(total - u_lo) + DEC_SLACK))) return rc;
@@ -1467,7 +1450,6 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
     for (auto& e : d.ev) CU_TRY(c, cudaEventCreate(&e));
     d.have_events = true;
   }
-  (void)dummy_cap;
   NvtxRange nvtx_copy("bgzf: H2D copy + inflate");
   // ---- windows of whole blocks, ~DEC_WINDOW_BYTES of file each
   struct Window { uint32_t b0, b1; uint64_t byte0, byte1; };
@@ -1540,35 +1522,21 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
   CU_TRY(c, cudaMemsetAsync(d.d_comp, 0, DEC_FRONT, c->stream));
   CU_TRY(c, cudaEventRecord(d.ev[1], c->stream));
   for (uint32_t t = 0; t < T; ++t) CU_TRY(c, cudaStreamWaitEvent(d.streams[t], d.ev[1], 0));
-  const bool serial = !inflate_per_window() && (windows.size() <= 1 || inflate_serial_requested());
-  const bool per_window = !serial && inflate_per_window();
-  const uint32_t NCS = 64;  // compute streams for the per-window launches
-  bool crc_pending = false;
-  InflateArgs persistent_args{};
-  if (per_window) {
-    CU_TRY(c, cudaFuncSetAttribute(kd_inflate_t1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM_BYTES));
-    while (d.cstreams.size() < std::min<size_t>(NCS, windows.size())) {
-      cudaStream_t cs;
-      CU_TRY(c, cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-      d.cstreams.push_back(cs);
-      cudaEvent_t e;
-      CU_TRY(c, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      d.cstream_done.push_back(e);
-    }
-    while (d.window_events.size() < windows.size()) {
-      cudaEvent_t e;
-      CU_TRY(c, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      d.window_events.push_back(e);
-    }
-    for (size_t k = 0; k < std::min<size_t>(NCS, windows.size()); ++k) CU_TRY(c, cudaStreamWaitEvent(d.cstreams[k], d.ev[1], 0));
-  } else if (!serial) {  // one persistent launch over every block; its warps wait for their block's window to arrive
+  // the InflateArgs of every inflate launch over blocks [b0, b1); the caller adds the block list or the arrival flags
+  auto inflate_args = [&](uint32_t b0, uint32_t b1, uint32_t* fail_count) {
     InflateArgs a{};
     a.comp = comp_base; a.coff = d.d_coff; a.clen = d.d_clen; a.isize = d.d_isize; a.uoff = d.d_ustart; a.scratch = d.d_t1_scratch;
+    a.b0 = b0; a.b1 = b1; a.out = infl_base; a.status = d.d_status; a.ticket = d.d_tickets; a.fail_count = fail_count;
+    return a;
+  };
+  const bool serial = windows.size() <= 1 || inflate_serial_requested();
+  bool crc_pending = false;
+  InflateArgs persistent_args{};
+  if (!serial) {  // one persistent launch over every block; its threads wait for their block's window to arrive
     // blocks before the one holding the first record are header text the host has already read: not inflated here
-    a.b0 = first_block; a.b1 = data_end; a.out = infl_base; a.status = d.d_status; a.ticket = d.d_tickets; a.fail_count = d.d_cnt + 0;
-    a.block_window = d.d_block_window; a.ready = d.d_tickets + 1;
-    persistent_args = a;
-    if ((rc = launch_inflate(c, a, c->stream, true, &crc_pending))) return rc;
+    persistent_args = inflate_args(first_block, data_end, d.d_cnt + 0);
+    persistent_args.block_window = d.d_block_window; persistent_args.ready = d.d_tickets + 1;
+    if ((rc = launch_inflate(c, persistent_args, c->stream, true, &crc_pending))) return rc;
   }
   std::atomic<size_t> next_window{0};
   std::atomic<int> first_err{0};
@@ -1602,22 +1570,7 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
           slot ^= 1;
         }
       }
-      if (per_window) {
-        // the window's blocks are inflated by their own launch, ordered behind the copy by an event; many windows' launches
-        // are in flight at once on the compute streams.  d_tickets[1 + w] (zeroed above) is that launch's block ticket.
-        cudaStream_t cs = d.cstreams[w % d.cstreams.size()];
-        if (!check(cudaEventRecord(d.window_events[w], st))) break;
-        if (!check(cudaStreamWaitEvent(cs, d.window_events[w], 0))) break;
-        InflateArgs a{};
-        a.comp = comp_base; a.coff = d.d_coff; a.clen = d.d_clen; a.isize = d.d_isize; a.uoff = d.d_ustart; a.scratch = d.d_t1_scratch;
-        a.b0 = win.b0; a.b1 = win.b1; a.out = infl_base; a.status = d.d_status; a.ticket = d.d_tickets + 1 + w; a.fail_count = d.d_cnt + 0;
-        const uint32_t nbw = win.b1 - win.b0;
-        kd_inflate_t1<<<(nbw + T1_THREADS - 1) / T1_THREADS, T1_THREADS, T1_SMEM_BYTES, cs>>>(a);
-        kd_crc32<<<std::max<uint32_t>(1, (nbw + 7) / 8), 256, 0, cs>>>(a);
-        if (!check(cudaGetLastError())) break;
-      } else if (!check(cudaMemcpyAsync(d.d_tickets + 1 + w, d.h_ones, 4, cudaMemcpyHostToDevice, st))) {  // window w has arrived
-        break;
-      }
+      if (!check(cudaMemcpyAsync(d.d_tickets + 1 + w, d.h_ones, 4, cudaMemcpyHostToDevice, st))) break;  // window w has arrived
     }
     check(cudaEventRecord(d.done_events[t], st));
   };
@@ -1633,10 +1586,7 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
   if (crc_pending && (rc = launch_crc32(c, persistent_args, c->stream))) return rc;  // every copy is enqueued: nothing left to hold up
   if (serial && !first_err.load()) {
     for (uint32_t t = 0; t < T; ++t) CU_TRY(c, cudaStreamWaitEvent(c->stream, d.done_events[t], 0));
-    InflateArgs a{};
-    a.comp = comp_base; a.coff = d.d_coff; a.clen = d.d_clen; a.isize = d.d_isize; a.uoff = d.d_ustart; a.scratch = d.d_t1_scratch;
-    a.b0 = first_block; a.b1 = data_end; a.out = infl_base; a.status = d.d_status; a.ticket = d.d_tickets; a.fail_count = d.d_cnt + 0;
-    if ((rc = launch_inflate(c, a, c->stream))) return rc;
+    if ((rc = launch_inflate(c, inflate_args(first_block, data_end, d.d_cnt + 0), c->stream))) return rc;
   }
   if (first_err.load()) {  // release the warps still waiting for windows that will never arrive
     cudaMemsetAsync(d.d_tickets + 1, 1, 4 * windows.size(), d.streams[0]);
@@ -1654,12 +1604,6 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
     fprintf(stderr, "#decode_h2d\twindows=%zu\tbytes=%llu\tcopy_streams_done_after_ms=%.1f (host clock from the end of the enqueue; enqueue took %.1f ms)\n",
             windows.size(), (unsigned long long)(byte_hi - byte_lo), wait_ms, copy_wall_ms);
   }
-  if (per_window) {
-    for (size_t k = 0; k < std::min<size_t>(NCS, windows.size()); ++k) {
-      CU_TRY(c, cudaEventRecord(d.cstream_done[k], d.cstreams[k]));
-      CU_TRY(c, cudaStreamWaitEvent(c->stream, d.cstream_done[k], 0));
-    }
-  }
   CU_TRY(c, cudaEventRecord(d.ev[2], c->stream));
   if (getenv("CMB_DECODE_PROFILE")) {  // debugging aid: the inflate kernel alone, all blocks resident, one launch
     CU_TRY(c, cudaStreamSynchronize(c->stream));
@@ -1667,11 +1611,8 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
     cudaEventCreate(&p0);
     cudaEventCreate(&p1);
     CU_TRY(c, cudaMemsetAsync(d.d_tickets, 0, 4, c->stream));
-    InflateArgs a{};
-    a.comp = comp_base; a.coff = d.d_coff; a.clen = d.d_clen; a.isize = d.d_isize; a.uoff = d.d_ustart; a.scratch = d.d_t1_scratch;
-    a.b0 = first_block; a.b1 = data_end; a.out = infl_base; a.status = d.d_status; a.ticket = d.d_tickets; a.fail_count = d.d_cnt + 8;
     cudaEventRecord(p0, c->stream);
-    if ((rc = launch_inflate(c, a, c->stream))) return rc;
+    if ((rc = launch_inflate(c, inflate_args(first_block, data_end, d.d_cnt + 8), c->stream))) return rc;
     cudaEventRecord(p1, c->stream);
     CU_TRY(c, cudaStreamSynchronize(c->stream));
     float ms = 0;
@@ -1712,10 +1653,8 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
         CU_TRY(c, cudaMemcpyAsync(d_list, again.data(), 4ull * again.size(), cudaMemcpyHostToDevice, c->stream));
         CU_TRY(c, cudaMemsetAsync(d.d_tickets, 0, 4, c->stream));
         CU_TRY(c, cudaMemsetAsync(d.d_cnt, 0, 4, c->stream));
-        InflateArgs a2{};
-        a2.comp = comp_base; a2.coff = d.d_coff; a2.clen = d.d_clen; a2.isize = d.d_isize; a2.uoff = d.d_ustart; a2.scratch = d.d_t1_scratch;
-        a2.b0 = 0; a2.b1 = (uint32_t)again.size(); a2.out = infl_base; a2.status = d.d_status; a2.ticket = d.d_tickets;
-        a2.fail_count = d.d_cnt + 0; a2.block_list = d_list;
+        InflateArgs a2 = inflate_args(0, (uint32_t)again.size(), d.d_cnt + 0);
+        a2.block_list = d_list;
         if ((rc = launch_inflate(c, a2, c->stream, false))) return rc;
         out->n_launches += 1;
         for (uint32_t b : again) status[b] = INF_OK;  // refreshed from the device below
@@ -1732,15 +1671,9 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
     for (uint32_t b = first_block; b < data_end; ++b) {
       if (status[b] == INF_OK) continue;
       const uint32_t isz = in->block_isize[b];
-      if (tmp.size() < isz) tmp.resize(isz);
-      inflateReset(&zs);
-      zs.next_in = const_cast<Bytef*>(in->data + in->block_coffset[b]);
-      zs.avail_in = in->block_clen[b];
-      zs.next_out = tmp.data();
-      zs.avail_out = isz;
       uint32_t want_crc;
       memcpy(&want_crc, in->data + in->block_coffset[b] + in->block_clen[b], 4);
-      if (inflate(&zs, Z_FINISH) != Z_STREAM_END || zs.avail_out != 0 || (uint32_t)crc32(0, tmp.data(), isz) != want_crc) {
+      if (!zlib_inflate_block(zs, in, b, tmp) || (uint32_t)crc32(0, tmp.data(), isz) != want_crc) {
         inflateEnd(&zs);
         return fail(c, CMB_E_DECLINED, "cmb_submit_bgzf: BGZF block %u does not inflate", b);
       }
@@ -1759,14 +1692,8 @@ int submit_bgzf_impl(cmb_ctx* c, const cmb_bgzf_input* in, cmb_bgzf_result* out,
     for (uint32_t b = first_block; b < data_end; ++b) {
       const uint32_t isz = in->block_isize[b];
       if (!isz) continue;
-      if (tmp.size() < isz) tmp.resize(isz);
-      inflateReset(&zs);
-      zs.next_in = const_cast<Bytef*>(in->data + in->block_coffset[b]);
-      zs.avail_in = in->block_clen[b];
-      zs.next_out = tmp.data();
-      zs.avail_out = isz;
-      const int zr = inflate(&zs, Z_FINISH);
-      if (zr != Z_STREAM_END || memcmp(tmp.data(), dev.data() + (ustart[b] - u_lo), isz) != 0) {
+      int zr = 0;
+      if (!zlib_inflate_block(zs, in, b, tmp, &zr) || memcmp(tmp.data(), dev.data() + (ustart[b] - u_lo), isz) != 0) {
         uint32_t k = 0;
         while (k < isz && tmp[k] == dev[ustart[b] - u_lo + k]) ++k;
         if (bad < 8) fprintf(stderr, "#decode_verify\tblock %u (clen %u isize %u): zlib rc %d, first difference at byte %u\n", b, in->block_clen[b], isz, zr, k);

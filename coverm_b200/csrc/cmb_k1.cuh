@@ -75,9 +75,6 @@ __device__ __forceinline__ bool read_pair_passes(const RecView& a, const RecView
 #ifndef CMB_K1_MINBLOCKS
 #define CMB_K1_MINBLOCKS 6
 #endif
-#ifndef CMB_K1_PREFETCH
-#define CMB_K1_PREFETCH 1  // issue the segment and first-interval loads right behind the column loads (one DRAM round trip less)
-#endif
 __global__ void __launch_bounds__(K1_THREADS, CMB_K1_MINBLOCKS) k1_filter_accumulate(const K1Args a) {
   const uint32_t i = blockIdx.x * K1_THREADS + threadIdx.x;
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -101,7 +98,6 @@ __global__ void __launch_bounds__(K1_THREADS, CMB_K1_MINBLOCKS) k1_filter_accumu
     ivb = a.iv_begin[i];
     ive = a.iv_begin[i + 1];
   }
-#if CMB_K1_PREFETCH
   // K1 is latency-bound (a thread's loads form the chain columns -> intervals -> segment table -> REDs).  The segment of a
   // record depends on its tid only and its first aligned block on iv_begin only, so both are requested here, before the
   // filter arithmetic and the block-wide sortedness scan, and are in registers by the time the events are added.
@@ -119,7 +115,6 @@ __global__ void __launch_bounds__(K1_THREADS, CMB_K1_MINBLOCKS) k1_filter_accumu
     pre_s = __ldg(a.iv_start + ivb);
     pre_n = __ldg(a.iv_len + ivb);
   }
-#endif
   const bool unmapped = r.flag & 0x4, secondary = r.flag & 0x100, supplementary = r.flag & 0x800, proper = r.flag & 0x2;
   // FlagFilter::passes, lib.rs:67-78
   const bool flag_pass = !(secondary && !p.include_secondary) && !(supplementary && !p.include_supplementary) &&
@@ -342,21 +337,10 @@ __global__ void __launch_bounds__(K1_THREADS, CMB_K1_MINBLOCKS) k1_filter_accumu
 
   // ---- delta events (contig.rs:171-186)
   if (mine) {
-    const uint32_t lc = (uint32_t)tid - a.tid_begin;
-    (void)lc;
-#if CMB_K1_PREFETCH
     const uint32_t L = pre_L, off0 = pre_off0, off1 = pre_off1;
-#else
-    const uint32_t L = a.len[lc], off0 = a.off_span[lc], off1 = a.off_span[lc + 1];
-#endif
     for (uint32_t k = ivb; k < ive; ++k) {
-#if CMB_K1_PREFETCH
       const int32_t s = k == ivb ? pre_s : a.iv_start[k];
       const uint32_t n = (uint32_t)(k == ivb ? pre_n : a.iv_len[k]);
-#else
-      const int32_t s = a.iv_start[k];
-      const uint32_t n = (uint32_t)a.iv_len[k];
-#endif
       if (s == INT_MIN) continue;  // CMB_IV_PAD: unused slot of the interval pool
       if (s < 0 || (uint32_t)s >= L) {  // `ups_and_downs[cursor] += 1` would panic
         err |= ERR_BOUNDS;

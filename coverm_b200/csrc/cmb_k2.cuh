@@ -1,11 +1,14 @@
 // K2: segmented prefix sum of the delta arena + every O(L) reduction of EST::add_contig, one pass, HBM-bound.
 //
-// Persistent CTAs (2 per SM, 8192/SPAN threads).  Each CTA claims 8192-element chunks with an atomic ticket and keeps a
-// 3-stage ring of 32 KB tiles in flight with TMA (cp.async.bulk.tensor.2d, 128B swizzle, mbarrier complete_tx).  A
-// thread owns one SPAN-element span (SPAN/4 x LDS.128, conflict-free through the swizzle); contigs start on span boundaries,
+// Persistent CTAs (CMB_K2_MINBLOCKS = 3 per SM, 256 threads).  CTA b works on the 8192-element chunks b, b + gridDim.x, ...
+// (a static schedule) and keeps a K2_STAGES-deep ring (2 by default) of 32 KB tiles in flight with TMA
+// (cp.async.bulk.tensor.2d, 128B swizzle, mbarrier complete_tx).  Since every thread knows its next chunk, the chunk's
+// metadata is loaded an iteration ahead and the contig lookup of a span runs while its tile is still arriving.  A thread
+// owns one 32-element span (one tile row: 8 x LDS.128, conflict-free through the swizzle) and re-zeroes the 16-byte units
+// of the arena that hold an event, so the arena is clean again for the next sample; contigs start on span boundaries,
 // so a span never straddles two contigs.  Running depth at a span = chunk carry (K1b) + segmented warp/CTA scan of the
 // span totals.  Depth is piecewise constant and deltas are sparse (~1-2 % of positions), so a thread only keeps the
-// span total and a SPAN-bit mask of its non-zero positions; covered bases, sum of depth and the depth histogram of the
+// span total and a 32-bit mask of its non-zero positions; covered bases, sum of depth and the depth histogram of the
 // end-trimmed window are then accumulated per RUN in a short loop over the set bits (the deltas are re-read from the
 // shared-memory tile, which stays resident until the next iteration's barrier).  The histogram lives in shared memory
 // per (contig slot, depth % 128) with the high depth bits as a tag, and is flushed as (depth,count) records while the
@@ -19,7 +22,6 @@ struct K2Args {
   const int32_t* carry_in;
   cmb_contig_stats* rows;
   uint32_t tid_begin, n_local, n_chunks, excl;
-  uint32_t* ticket;
   int32_t* arena;
   uint2* rec;
   uint32_t rec_capacity;
@@ -33,52 +35,28 @@ struct K2Args {
 };
 
 constexpr uint32_t K2_SMEM_STAGE_BYTES = K2_STAGES * CHUNK_BYTES;
-#if CMB_SPAN > 32
-typedef unsigned long long evmask_t;  // one bit per element of a span
-__device__ __forceinline__ uint32_t ev_first(evmask_t m) { return (uint32_t)__ffsll((long long)m) - 1; }
-#else
-typedef uint32_t evmask_t;
-__device__ __forceinline__ uint32_t ev_first(evmask_t m) { return (uint32_t)__ffs((int)m) - 1; }
-#endif
-static_assert(SPAN == 16 || SPAN == 32 || SPAN == 64, "a span is 16, 32 or 64 elements");
-constexpr uint32_t K2_SMEM_MISC = 64 /*barriers + tickets*/ + 2 * K2_WARPS * 8 /*warp aggregates, double-buffered*/;
+constexpr uint32_t K2_SMEM_MISC = 64 /*barriers*/ + 2 * K2_WARPS * 8 /*warp aggregates, double-buffered*/;
 constexpr uint32_t K2_SMEM_BYTES_HIST = K2_SMEM_STAGE_BYTES + K2_SMEM_MISC + 2 * HIST_TOTAL * 4;
 constexpr uint32_t K2_SMEM_BYTES_NOHIST = K2_SMEM_STAGE_BYTES + K2_SMEM_MISC;
 
-template <bool HIST, bool CLEAN>
+template <bool HIST>
 __global__ void __launch_bounds__(K2_THREADS, CMB_K2_MINBLOCKS) k2_scan_reduce(const __grid_constant__ CUtensorMap tmap, const K2Args a) {
   extern __shared__ __align__(1024) uint8_t smem[];  // stage tiles need the 1024 B swizzle-atom alignment
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + K2_SMEM_STAGE_BYTES);
-  uint32_t* s_chunk = reinterpret_cast<uint32_t*>(full + K2_STAGES);
   int2* wagg2 = reinterpret_cast<int2*>(smem + K2_SMEM_STAGE_BYTES + 64);
   uint32_t* hist2 = reinterpret_cast<uint32_t*>(wagg2 + 2 * K2_WARPS);
 
   const uint32_t t = threadIdx.x, lane = t & 31, warp = t >> 5;
 
-#if CMB_K2_STATIC
   // Static schedule: iteration i of CTA b works on chunk b + i * gridDim.x.  Every thread knows its next chunk, so the chunk's
   // metadata (first / last contig, carry-in) is requested one iteration ahead and the dependent lookups (contig of the span,
-  // its start and length) can start before the tile has even arrived; no ticket atomics, no ticket hand-over through shared memory.
+  // its start and length) can start before the tile has even arrived.
   auto chunk_of = [&](uint32_t i) -> uint32_t { return blockIdx.x + i * gridDim.x; };
-  auto issue_static = [&](uint32_t s, uint32_t ck) {  // thread 0: start the TMA load of chunk ck into stage s
+  auto issue = [&](uint32_t s, uint32_t ck) {  // thread 0: start the TMA load of chunk ck into stage s
     if (ck < a.n_chunks) {
       const uint32_t bar = smem_u32(full + s);
       mbar_arrive_expect_tx(bar, CHUNK_BYTES);
       tma_load_2d(smem_u32(smem + s * CHUNK_BYTES), &tmap, 0, (int32_t)(ck * CHUNK_ROWS), bar);
-    }
-  };
-#endif
-  auto issue = [&](uint32_t s) {  // thread 0: claim the next chunk and start its TMA load into stage s
-    // The ticket travels with the barrier phase: it is written before the arrive (release) and read by the consumers
-    // after their wait (acquire), so a stage may be refilled for the very next iteration (2-stage rings).
-    const uint32_t tk = atomicAdd(a.ticket, 1u);
-    s_chunk[s] = tk;
-    const uint32_t bar = smem_u32(full + s);
-    if (tk < a.n_chunks) {
-      mbar_arrive_expect_tx(bar, CHUNK_BYTES);
-      tma_load_2d(smem_u32(smem + s * CHUNK_BYTES), &tmap, 0, (int32_t)(tk * CHUNK_ROWS), bar);
-    } else {
-      mbar_arrive(bar);  // no more chunks: complete the phase so that the consumers wake up and see the end ticket
     }
   };
 
@@ -122,29 +100,20 @@ __global__ void __launch_bounds__(K2_THREADS, CMB_K2_MINBLOCKS) k2_scan_reduce(c
     for (uint32_t b = t; b < 2 * HIST_TOTAL; b += K2_THREADS) hist2[b] = 0;
   __syncthreads();
   if (t == 0)
-#if CMB_K2_STATIC
-    for (uint32_t s = 0; s < K2_STAGES; ++s) issue_static(s, chunk_of(s));
-#else
-    for (uint32_t s = 0; s < K2_STAGES; ++s) issue(s);
-#endif
+    for (uint32_t s = 0; s < K2_STAGES; ++s) issue(s, chunk_of(s));
   __syncthreads();
 
-  constexpr uint32_t UNITS = SPAN / 4;                 // 16-byte units per span
-  const uint32_t row = (t * SPAN) / ROW_ELEMS;          // first 128-byte tile row of this thread's span
-  const uint32_t u0 = (t * UNITS) % (ROW_ELEMS / 4);    // its first unit within the row (0 unless SPAN < 32)
-  // A span of 64 is two tile rows, so the eight lanes of an LDS.128 phase sit on rows 0,2,..,14 and the 128B swizzle alone
-  // leaves lanes l and l+4 on the same banks.  Lanes 4..7 of every eight therefore visit their units in pairs swapped
-  // (unit j^1 when the others read unit j); the event mask is put back in position order after the loop.
-  const uint32_t swp = SPAN > 32 ? ((t >> 2) & 1u) : 0u;
+  static_assert(SPAN == ROW_ELEMS, "a span is one 128-byte tile row");
+  constexpr uint32_t UNITS = SPAN / 4;  // 16-byte units per span
+  const uint32_t row = t;               // the tile row of this thread's span
   // byte offset inside a stage tile of element e of this thread's span
   auto elem_off = [&](uint32_t e) -> uint32_t {
-    const uint32_t idx = u0 + (e >> 2);
+    const uint32_t idx = e >> 2;
     const uint32_t r = row + (idx >> 3);
     return r * 128 + (((idx & 7) ^ (r & 7)) << 4) + ((e & 3) << 2);
   };
   const uint32_t E = a.excl;
   uint32_t prev_chunk = 0, prev_slots = 0;
-#if CMB_K2_STATIC
   uint32_t n_cf = 0, n_cl = 0;  // metadata of the NEXT iteration's chunk, requested an iteration ahead
   int n_cin = 0;
   if (chunk_of(0) < a.n_chunks) {
@@ -152,12 +121,10 @@ __global__ void __launch_bounds__(K2_THREADS, CMB_K2_MINBLOCKS) k2_scan_reduce(c
     n_cl = __ldg(a.chunk_first + chunk_of(0) + 1);
     n_cin = __ldg(a.carry_in + chunk_of(0));
   }
-#endif
   uint32_t it = 0;
 
   for (;; ++it) {
     const uint32_t s = it % K2_STAGES;
-#if CMB_K2_STATIC
     const uint32_t chunk = chunk_of(it);
     if (chunk >= a.n_chunks) break;
     const uint32_t cf = n_cf, cl = n_cl;
@@ -185,91 +152,26 @@ __global__ void __launch_bounds__(K2_THREADS, CMB_K2_MINBLOCKS) k2_scan_reduce(c
     const uint32_t cstart = __ldg(a.off_span + c);
     const uint32_t L = __ldg(a.len + c);
     mbar_wait(smem_u32(full + s), (it / K2_STAGES) & 1);
-#else
-    mbar_wait(smem_u32(full + s), (it / K2_STAGES) & 1);
-    const uint32_t chunk = *(volatile uint32_t*)(s_chunk + s);
-    if (chunk >= a.n_chunks) break;
-#endif
     int2* wagg = wagg2 + (it & 1) * K2_WARPS;
     uint32_t* hist = hist2 + (it & 1) * HIST_TOTAL;
 
     // ---- SPAN consecutive deltas per thread: LDS.128s through the 128B swizzle (conflict-free).
     //      Only their sum and the mask of non-zero positions stay in registers.
     const uint8_t* tilep = smem + s * CHUNK_BYTES;
-#if CMB_K2_COOP && CMB_SPAN == 32
-    const uint8_t* rowp = tilep + row * 128;
-#endif
-#if !CMB_K2_STATIC
-    const uint32_t span = chunk * CHUNK_SPANS + t;
-#endif
     int total = 0;
-    evmask_t ev = 0;
-#if CMB_K2_COOP && CMB_SPAN == 32
-    {
-      // Deltas are sparse (under 1 % of the positions; about three spans in four hold none), but a branch per thread saves
-      // nothing in SIMT -- some lane of the warp always has events.  So the work is compacted across the warp: every lane only
-      // ORs its 32 values together (a span is one 128-byte tile row); then the WARP visits each non-empty span of its lanes
-      // once, lane e taking element e of that row: one conflict-free LDS.32, one ballot (the non-zero mask) and one REDUX (the
-      // span total) replace the owner's thirty-two compares and adds, and the re-zeroing stores go out from the lanes that
-      // saw the events.
-      uint32_t any = 0;
-#pragma unroll
-      for (uint32_t j = 0; j < UNITS; ++j) {
-        const int4 q = *reinterpret_cast<const int4*>(rowp + ((j ^ (row & 7)) << 4));  // every unit once, bank-conflict-free
-        any |= (uint32_t)((q.x | q.y) | (q.z | q.w));
-      }
-      uint32_t busy = __ballot_sync(FULL, any != 0);
-      const uint8_t* tile = smem + s * CHUNK_BYTES;
-      while (busy) {
-        const uint32_t src = (uint32_t)__ffs(busy) - 1;
-        busy &= busy - 1;
-        const uint32_t r2 = (t & ~31u) + src;  // tile row == span of lane `src`
-        const int v = *reinterpret_cast<const int*>(tile + r2 * 128 + (((lane >> 2) ^ (r2 & 7)) << 4) + ((lane & 3) << 2));
-        const uint32_t m = __ballot_sync(FULL, v != 0);
-        const int sum = __reduce_add_sync(FULL, v);
-        if (lane == src) {
-          total = sum;
-          ev = m;
-        }
-        if (CLEAN && v != 0) a.arena[((uint64_t)chunk * CHUNK_SPANS + r2) * SPAN + lane] = 0;
-      }
-    }
-#else
+    uint32_t ev = 0;
     {
       int4* g = reinterpret_cast<int4*>(a.arena + (uint64_t)span * SPAN);
-      int4* g_even = g + swp;  // unit j^swp == j + swp for even j, j - swp for odd j
-      int4* g_odd = g - swp;
 #pragma unroll
       for (uint32_t j = 0; j < UNITS; ++j) {
-        const uint32_t r = row + ((u0 + j) >> 3);
-        const uint32_t unit = (((u0 + j) & 7) ^ swp) ^ (r & 7);  // unit j^swp of the span, through the swizzle of its row
-        const int4 q = *reinterpret_cast<const int4*>(tilep + r * 128 + unit * 16);
+        const int4 q = *reinterpret_cast<const int4*>(tilep + row * 128 + ((j ^ (row & 7)) << 4));
         const uint32_t e4 = (q.x != 0 ? 1u : 0u) | (q.y != 0 ? 2u : 0u) | (q.z != 0 ? 4u : 0u) | (q.w != 0 ? 8u : 0u);
         total += (q.x + q.y) + (q.z + q.w);
-        ev |= (evmask_t)e4 << (4 * j);
-        if (CLEAN && e4) ((j & 1) ? g_odd : g_even)[j] = make_int4(0, 0, 0, 0);  // re-zero only the 16 B units that hold an event
-      }
-      if (SPAN > 32 && swp) {  // back to position order: swap neighbouring nibbles
-        constexpr evmask_t LO = (evmask_t)0x0f0f0f0f0f0f0f0full;
-        ev = ((ev & LO) << 4) | ((ev >> 4) & LO);
+        ev |= e4 << (4 * j);
+        if (e4) g[j] = make_int4(0, 0, 0, 0);  // re-zero only the 16 B units that hold an event
       }
     }
-#endif
 
-    // ---- which contig owns this span
-#if !CMB_K2_STATIC
-    const uint32_t cf = __ldg(a.chunk_first + chunk);
-    const uint32_t cl = __ldg(a.chunk_first + chunk + 1);
-    uint32_t lo = cf, hi = cl;
-    while (lo < hi) {
-      const uint32_t mid = (lo + hi + 1) >> 1;
-      if (__ldg(a.off_span + mid) <= span) lo = mid;
-      else hi = mid - 1;
-    }
-    const uint32_t c = lo;
-    const uint32_t cstart = __ldg(a.off_span + c);
-    const uint32_t L = __ldg(a.len + c);
-#endif
     const bool is_head = span == cstart;
     const uint32_t rel = (span - cstart) * SPAN;  // position in the contig of the span's first element
     const uint32_t n_in = rel >= L ? 0u : min(SPAN, L - rel);
@@ -301,11 +203,7 @@ __global__ void __launch_bounds__(K2_THREADS, CMB_K2_MINBLOCKS) k2_scan_reduce(c
     if (lane == 31) wagg[warp] = make_int2(val, flg);
     __syncthreads();  // warp aggregates visible; the previous iteration's tile and histogram adds are complete
     if (it > 0) {
-#if CMB_K2_STATIC
-      if (t == 0) issue_static((it - 1) % K2_STAGES, chunk_of(it - 1 + K2_STAGES));  // refill the tile of the previous iteration
-#else
-      if (t == 0) issue((it - 1) % K2_STAGES);  // refill the tile of the previous iteration (read until this barrier)
-#endif
+      if (t == 0) issue((it - 1) % K2_STAGES, chunk_of(it - 1 + K2_STAGES));  // refill the tile of the previous iteration
       if (HIST) flush_hist(hist2 + ((it & 1) ^ 1) * HIST_TOTAL, prev_chunk, prev_slots);
     }
 
@@ -331,9 +229,6 @@ __global__ void __launch_bounds__(K2_THREADS, CMB_K2_MINBLOCKS) k2_scan_reduce(c
         wf = 0;
       }
     }
-#if !CMB_K2_STATIC
-    const int cin = __ldg(a.carry_in + chunk);
-#endif
     int carry;
     if (is_head) carry = 0;
     else if (pflg) carry = pval;
@@ -389,9 +284,9 @@ __global__ void __launch_bounds__(K2_THREADS, CMB_K2_MINBLOCKS) k2_scan_reduce(c
     if (ev) {
       int depth = carry;
       uint32_t from = 0;
-      evmask_t m = ev;
+      uint32_t m = ev;
       while (m) {
-        const uint32_t j = ev_first(m);
+        const uint32_t j = (uint32_t)__ffs((int)m) - 1;
         m &= m - 1;
         close_run(depth, from, j);
         depth += *reinterpret_cast<const int*>(tilep + elem_off(j));  // the delta at position j

@@ -37,7 +37,7 @@ static const uint8_t c_clen_order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4
 struct InflateArgs {
   const uint8_t* comp; const uint64_t* coff; const uint32_t* clen; const uint32_t* isize; const uint64_t* uoff;
   uint32_t b0, b1; uint8_t* out; uint32_t* status; uint32_t* ticket; uint32_t* fail_count;
-  const uint32_t* block_window; const uint32_t* ready; uint32_t lane_limit, static_first;
+  const uint32_t* block_window; const uint32_t* ready; uint32_t lane_limit;
   const uint32_t* block_list; uint8_t* scratch;
 };
 uint8_t t1_smem[4096];

@@ -156,16 +156,16 @@ def test_host_decode_path_matches_oracle(synth, which, argv):
     assert any(l.startswith("#pipeline") for l in g.stderr.splitlines())
 
 
-INFLATE_MODES = [(k, m) for k in ("t1", "g8", "w1") for m in ("persistent", "serial")] + [("t1", "windows")]
+INFLATE_MODES = [(k, m) for k in ("t1", "g8", "w1") for m in ("persistent", "serial")]
 
 
 @pytest.mark.parametrize("kernel,mode", INFLATE_MODES, ids=[f"{k}-{m}" for k, m in INFLATE_MODES])
 def test_every_inflate_kernel_and_launch_mode_matches_zlib(synth, kernel, mode):
-    """The three inflate kernels (thread / eight lanes / warp per block) under the three launch disciplines: one persistent launch
-    whose lanes wait for their window's arrival flag (64 KB windows here, so that a small file spans many), one launch ordered
-    behind all the copies (what runs under ncu / compute-sanitizer and for single-window files), one launch per window."""
+    """The three inflate kernels (thread / eight lanes / warp per block) under the two launch disciplines: one persistent launch
+    whose lanes wait for their window's arrival flag (64 KB windows here, so that a small file spans many), and one launch
+    ordered behind all the copies (what runs under ncu / compute-sanitizer and for single-window files)."""
     env = {"CMB_PIPELINE_STATS": "1", "CMB_DECODE_VERIFY": "1", "CMB_INFLATE": kernel, "CMB_DECODE_WINDOW_KB": "64",
-           "CMB_INFLATE_SERIAL": "1" if mode == "serial" else "0", "CMB_INFLATE_WINDOWS": "1" if mode == "windows" else "0"}
+           "CMB_INFLATE_SERIAL": "1" if mode == "serial" else "0"}
     for which in ("small", "mags"):
         g = _assert_same(["contig", "-m", "mean", "trimmed_mean", "count", "-b", synth[which]], env=env)
         st = _decode_stats(g)
